@@ -27,6 +27,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True        # the tree the bench runs from may be read-only: nothing is written there
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -39,7 +40,8 @@ METRIC = "stereo frames/sec at 1241x376, 2000 feats; LK kernel HBM GB/s vs roofl
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="steps in a timed block; each path's block is timed 5 times and the median block reported")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--units", type=int, default=8, help="independent stereo pairs per step per GPU")
@@ -52,6 +54,9 @@ def parse():
     ap.add_argument("--width", type=int, default=W_IMG)
     ap.add_argument("--height", type=int, default=H_IMG)
     ap.add_argument("--calib", default="kitti", choices=["kitti", "zed"], help="intrinsics of the synthetic rig")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last resident and the last end-to-end step returned as "
+                         "DIR/<name>.npy (rank 0's units, at most 64 MB)")
     return ap.parse_args()
 
 
@@ -435,6 +440,36 @@ def check_against_oracle(got, res, ref):
     return bad
 
 
+DUMP_BYTES = 64 << 20
+RECORD_COUNTS = ("n_features", "n_detected", "n_tracked", "n_valid", "n_inliers", "ransac_iters", "pnp_status")
+POINT_LISTS = (("l0", np.float32), ("r0", np.float32), ("l1", np.float32), ("r1", np.float32), ("X", np.float32),
+               ("kept_idx", np.float64), ("inliers", np.float64))
+
+
+def dump_outputs(out_dir, res, res_e2e, outputs, features):
+    """What the last step of the timed paths returned, one DIR/<name>.npy per array (float64; point lists float32):
+      units                  the units written (indices into the step's units)
+      resident_*, e2e_*      their result records: counts (columns as RECORD_COUNTS), rvec, tvec, R
+      e2e_l0 ... e2e_inliers their point lists from the end-to-end path, concatenated in unit order (a unit has
+                             e2e_counts[:, 3] = n_valid rows of each list but inliers, and e2e_counts[:, 4] of those)
+    When the worst case of all units exceeds DUMP_BYTES, a fixed seeded sample of the units is written."""
+    per_unit = 60 * features + 360        # n_valid <= features rows of all lists (60 B), two records, the unit index
+    units = np.arange(len(res))
+    if len(units) * per_unit > DUMP_BYTES:
+        units = np.sort(np.random.default_rng(0).choice(len(units), DUMP_BYTES // per_unit, replace=False))
+    arrays = {"units": units.astype(np.float64)}
+    for prefix, recs in (("resident", res), ("e2e", res_e2e)):
+        recs = [recs[u] for u in units]
+        arrays[prefix + "_counts"] = np.array([[r[k] for k in RECORD_COUNTS] for r in recs], np.float64).reshape(-1, len(RECORD_COUNTS))
+        for k, shape in (("rvec", (3,)), ("tvec", (3,)), ("R", (3, 3))):
+            arrays[f"{prefix}_{k}"] = np.array([r[k] for r in recs], np.float64).reshape((-1,) + shape)
+    for k, dt in POINT_LISTS:
+        arrays["e2e_" + k] = np.concatenate([np.asarray(outputs[u][k], dt) for u in units])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 class Point:
     """One workload point (image size, features, units per step) measured on a context: the pipelined resident pass
     (`value`), the LK kernel alone on one stream (roofline) and the pipelined end-to-end pass with pinned host images in
@@ -720,6 +755,8 @@ def main():
     ref = reference_unit_outputs(units[last_slot_unit], args.features)
     bad = check_against_oracle(pt.last_outputs[last_slot_unit], res_e2e[last_slot_unit], ref)
     oracle_s = time.perf_counter() - t_or
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, res_e2e, pt.last_outputs, args.features)
     gather_ok = True
     if world > 1 and getattr(pt, "tables", None):          # the gathered table holds this rank's records where they belong
         last = pt.tables[-1]

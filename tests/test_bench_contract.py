@@ -73,3 +73,48 @@ def test_native_gather_bookkeeping_never_exceeds_the_library_depth():
     tables = g.drain()
     assert tables == list(range(20)) and ctx.posted == ctx.waited == 20 and ctx.max_out == VO_DIST_DEPTH
     assert g.drain() == []
+
+
+def test_dump_outputs_writes_float_arrays_within_the_budget(tmp_path):
+    """bench.dump_outputs (--dump-outputs DIR): float32 / float64 .npy files only, the point lists concatenated in unit order
+    as the records count them, and a step whose worst case exceeds the budget cut to the same seeded sample of units."""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+
+    rng = np.random.default_rng(5)
+    recs, outs = [], []
+    for u in range(40):
+        nv = int(rng.integers(0, 50))
+        ni = int(rng.integers(0, nv + 1))
+        recs.append(dict(n_features=50, n_detected=60 + u, n_tracked=nv + 1, n_valid=nv, n_inliers=ni, ransac_iters=u, pnp_status=0,
+                         rvec=rng.normal(size=3), tvec=rng.normal(size=3), R=rng.normal(size=(3, 3))))
+        outs.append(dict(l0=rng.random((nv, 2), np.float32), r0=rng.random((nv, 2), np.float32), l1=rng.random((nv, 2), np.float32),
+                         r1=rng.random((nv, 2), np.float32), X=rng.random((nv, 3), np.float32),
+                         kept_idx=np.sort(rng.choice(50, nv, replace=False)).astype(np.int32), inliers=np.arange(ni, dtype=np.int32)))
+
+    def load(d):
+        files = sorted(os.listdir(d))
+        assert all(f.endswith(".npy") for f in files)
+        return {f[:-4]: np.load(os.path.join(d, f)) for f in files}
+
+    bench.dump_outputs(str(tmp_path / "all"), recs, recs, outs, 50)
+    a = load(tmp_path / "all")
+    names = {"units"} | {p + k for p in ("resident_", "e2e_") for k in ("counts", "rvec", "tvec", "R")} | {"e2e_" + k for k, _ in bench.POINT_LISTS}
+    assert set(a) == names and all(x.dtype in (np.float32, np.float64) for x in a.values())
+    assert np.array_equal(a["units"], np.arange(40)) and a["e2e_counts"].shape == (40, 7) and a["e2e_R"].shape == (40, 3, 3)
+    assert np.array_equal(a["resident_counts"][:, 3], [r["n_valid"] for r in recs])
+    for k, dt in bench.POINT_LISTS:
+        assert np.array_equal(a["e2e_" + k], np.concatenate([o[k] for o in outs]).astype(dt)), k
+
+    bench.DUMP_BYTES = 10 * (60 * 50 + 360)         # room for the worst case of 10 units
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), recs, recs, outs, 50)
+    s1, s2 = load(tmp_path / "s1"), load(tmp_path / "s2")
+    assert all(np.array_equal(s1[k], s2[k]) for k in names)
+    units = s1["units"].astype(int)
+    assert len(units) == 10 and np.all(np.diff(units) > 0) and sum(x.nbytes for x in s1.values()) <= bench.DUMP_BYTES
+    assert np.array_equal(s1["e2e_tvec"], [recs[u]["tvec"] for u in units])
+    assert np.array_equal(s1["e2e_l1"], np.concatenate([outs[u]["l1"] for u in units]))
